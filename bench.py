@@ -39,6 +39,7 @@ sys.path.insert(0, str(REPO))
 SEQ_LEN = 4096
 METRIC = "tokens/sec (Qwen3-8B FSDP2 bf16 seq4096)"
 CPU_SAMPLE_TOKENS = 256  # the bounded CPU sample: one definition for `cpu_baseline` and `--impl reference`
+DUMP_SAMPLE = 4096  # --dump-outputs: sampled elements per parameter (Qwen3-8B: 399 parameters, 5.4 MB in all)
 
 # DRAM bytes per launch (read + write) of the three attention kernels at T=4096, 32/8 heads, D=128, from ncu --set full
 # (profiles/r02_topkernels_ncu.txt: attn_bwd_dkdv_tc_kernel, attn_bwd_dq_n128_kernel, attn_fwd_tc_kernel<W8>)
@@ -159,6 +160,30 @@ def run_reference(args) -> None:
     print(json.dumps(out), flush=True)
 
 
+def dump_outputs(out_dir: Path, model, opt, loss: float, grad_norm) -> None:
+    """Write what the last timed step handed back as float arrays, for output-for-output comparison of two builds:
+    ``loss.npy`` and ``grad_norm.npy`` (float64, shape [1]) and ``params_sample.npy`` (float32), the updated parameters
+    (the optimizer's fp32 masters where it keeps them) at DUMP_SAMPLE seeded positions each, in ``named_parameters``
+    order. Under FSDP the sample is this rank's shard."""
+    import numpy as np
+    import torch
+    from torch.distributed.tensor import DTensor
+
+    g = torch.Generator().manual_seed(0)
+    parts = []
+    with torch.no_grad():
+        for _, p in model.named_parameters():
+            t = opt.state[p].get("master", p) if p in opt.state else p
+            t = (t.to_local() if isinstance(t, DTensor) else t).reshape(-1)
+            if t.numel():
+                idx = torch.randint(0, t.numel(), (min(DUMP_SAMPLE, t.numel()),), generator=g)
+                parts.append(t[idx.to(t.device)].float().cpu())
+    out_dir.mkdir(parents=True, exist_ok=True)
+    np.save(out_dir / "loss.npy", np.array([loss], dtype=np.float64))
+    np.save(out_dir / "grad_norm.npy", np.array([float(grad_norm)], dtype=np.float64))
+    np.save(out_dir / "params_sample.npy", torch.cat(parts).numpy())
+
+
 # ------------------------------------------------------------------------------------------------
 def run_b200(args) -> None:
     import torch
@@ -270,6 +295,7 @@ def run_b200(args) -> None:
     h2d_bytes = sum(t.numel() * t.element_size() for t in host[0])
     n_valid_local = [int((h[1] != -100).sum()) for h in host]
     sp_group = getattr(model, "sp_group", None)
+    last_grad_norm = [None]  # device scalar of the latest step, kept for --dump-outputs
 
     def step(batch, i=0):
         ids, shift, pos = batch
@@ -278,10 +304,10 @@ def run_b200(args) -> None:
             loss = loss * (n_valid_local[i % nbuf] * sp / float(seq_len - 1))
         loss.backward()
         if fold_clip:
-            _, coef = clip_grad_norm(model, 1.0, return_coef=True)  # veomni_clip_grad_norm semantics; the scaling pass
-            opt.step(grad_scale=coef)                               # is folded into the AdamW kernel
+            last_grad_norm[0], coef = clip_grad_norm(model, 1.0, return_coef=True)  # veomni_clip_grad_norm semantics; the
+            opt.step(grad_scale=coef)                                                # scaling pass is folded into AdamW
         else:
-            clip_grad_norm(model, 1.0)
+            last_grad_norm[0] = clip_grad_norm(model, 1.0)
             opt.step()
         opt.zero_grad(set_to_none=True)
         return loss
@@ -340,6 +366,8 @@ def run_b200(args) -> None:
     aprof, vattn.PROFILE = vattn.PROFILE, None
     cprof, prof.ACTIVE = prof.ACTIVE, None
     torch.cuda.synchronize()
+    if args.dump_outputs and rank == 0:  # before the e2e pass below moves the weights on
+        dump_outputs(Path(args.dump_outputs), model, opt, loss_dev, last_grad_norm[0])
     prof_ms = {k: [a.elapsed_time(b) for a, b in v] for k, v in aprof.items()}
     comm_stats = prof.summarize(cprof)
     ms_e2e, loss_e2e = timed(args.steps, e2e=True)
@@ -516,7 +544,11 @@ def main():
     ap.add_argument("--skip-parity", action="store_true", help="skip the multi-GPU parity stage")
     ap.add_argument("--skip-ab", action="store_true", help="skip the NCCL-comm A/B side measurement")
     ap.add_argument("--torch-profile", default="", help="debug: write a torch.profiler kernel table of one extra step")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 training step")
     if args.impl == "reference":
         run_reference(args)
     else:

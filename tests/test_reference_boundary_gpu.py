@@ -1,108 +1,76 @@
-"""The REAL reference, on the GPU, through the drop-in boundary.
+"""The REAL reference, on the GPU, through the drop-in boundary — against what its stock ops compute.
 
-``baseline/_ref`` holds an unmodified install of VeOmni (recipe: ``tools/install_reference.sh`` =
-``pip install --no-index --no-build-isolation --no-deps --target baseline/_ref /root/reference``; git-ignored, it travels
-to the GPU box with the snapshot).  The test builds the reference's OWN patched models with its OWN
-``build_foundation_model`` -> ``_bind_veomni_ops`` (veomni/models/auto.py:63-103, 106-...), once on the reference's stock
-ops and once with ``b200`` selected for every op this package registers (``veomni_b200.registry.register()``:
-``rms_norm`` / ``rotary_pos_emb`` / ``swiglu_mlp`` / ``cross_entropy_loss`` / ``moe_experts`` OpSlots, the HF
-attention table entry and the fused-MoE pointer), runs the same packed batch through both and applies the reference's
-own cross-backend bar: loss and grad-norm within 1e-2 relative (tests/models/test_models_patch.py:327-329).
+tests/golden/reference_boundary.json (tests/golden/make_reference_boundary.py) holds the loss and global gradient norm
+of the unmodified reference's toy Qwen3 and Qwen3-MoE (its ``build_foundation_model`` -> ``_bind_veomni_ops``, bf16 on a
+B200, eager ops and flash-attn-2 varlen attention) for the weights and packed 3-sequence batch that module draws.
 
-Skips only when the install is absent or cannot be imported on the box.
+* ``test_reference_models_with_b200_ops_match_reference_stock_ops``: the reference package that ``build()`` places in
+  ``oracle/_ref`` (oracle/build_ref.py) builds the same models again, with ``b200`` selected for every op
+  ``veomni_b200.registry.register()`` installs (``rms_norm`` / ``rotary_pos_emb`` / ``swiglu_mlp`` /
+  ``cross_entropy_loss`` / ``moe_experts`` OpSlots, the HF attention table entry and the fused-MoE pointer). Skips only
+  when ``oracle/_ref`` holds no reference package.
+* ``test_host_models_match_reference_stock_ops``: the host mirror of the same models on the veomni_b200 kernels.
+
+Both apply the reference's own cross-backend bar: loss and grad-norm within 1e-2 relative
+(tests/models/test_models_patch.py:327-329).
 """
+import importlib.util
 import json
 import sys
-import tempfile
 from pathlib import Path
 
 import pytest
 import torch
 
+from oracle.build_ref import REF_DIR
+
 pytestmark = pytest.mark.gpu
-REPO = Path(__file__).resolve().parent.parent
-REF = REPO / "baseline" / "_ref"
-
-QWEN3_TOY = dict(hidden_size=1024, intermediate_size=2048, num_hidden_layers=2, num_attention_heads=8, num_key_value_heads=2,
-                 head_dim=128, vocab_size=2048, max_position_embeddings=4096, rms_norm_eps=1e-6, tie_word_embeddings=False,
-                 rope_theta=1000000.0, architectures=["Qwen3ForCausalLM"], model_type="qwen3")
-QWEN3_MOE_TOY = dict(hidden_size=1024, intermediate_size=2048, moe_intermediate_size=256, num_experts=8, num_experts_per_tok=2,
-                     num_hidden_layers=2, num_attention_heads=8, num_key_value_heads=2, head_dim=128, vocab_size=2048,
-                     max_position_embeddings=4096, rms_norm_eps=1e-6, tie_word_embeddings=False, rope_theta=1000000.0,
-                     decoder_sparse_step=1, mlp_only_layers=[], norm_topk_prob=True, output_router_logits=False,
-                     router_aux_loss_coef=0.0, architectures=["Qwen3MoeForCausalLM"], model_type="qwen3_moe")
+GOLDEN = Path(__file__).resolve().parent / "golden"
+_spec = importlib.util.spec_from_file_location("make_reference_boundary", GOLDEN / "make_reference_boundary.py")
+MRB = importlib.util.module_from_spec(_spec)
+_spec.loader.exec_module(MRB)
+CASES = [("qwen3", MRB.QWEN3_TOY), ("qwen3_moe", MRB.QWEN3_MOE_TOY)]
 
 
-def _reference():
-    if not (REF / "veomni").is_dir():
-        pytest.skip("baseline/_ref is absent: run tools/install_reference.sh in the authoring container")
-    if str(REF) not in sys.path:
-        sys.path.insert(0, str(REF))
-    try:
-        from veomni.arguments.arguments_types import OpsImplementationConfig
-        from veomni.models import build_foundation_model
-    except Exception as ex:  # noqa: BLE001
-        pytest.skip(f"the reference install cannot be imported here: {type(ex).__name__}: {ex}")
-    return build_foundation_model, OpsImplementationConfig
+def _check(name: str, loss: float, gn: float, launches: int) -> None:
+    ref = json.loads((GOLDEN / "reference_boundary.json").read_text())[name]
+    print(json.dumps({"model": name, "loss_ref": ref["loss"], "loss_b200": loss, "grad_norm_ref": ref["grad_norm"],
+                      "grad_norm_b200": gn, "b200_kernel_launches": launches}))
+    assert launches > 0, "not a single veomni_b200 kernel launched"
+    assert abs(loss - ref["loss"]) / abs(ref["loss"]) < 1e-2, (loss, ref["loss"])
+    assert abs(gn - ref["grad_norm"]) / ref["grad_norm"] < 1e-2, (gn, ref["grad_norm"])
 
 
-def _ops(cls, **kw):
-    base = dict(attn_implementation="flash_attention_2", moe_implementation="eager", cross_entropy_loss_implementation="eager",
-                rms_norm_implementation="eager", swiglu_mlp_implementation="eager", rotary_pos_emb_implementation="eager",
-                load_balancing_loss_implementation="eager", rms_norm_gated_implementation="eager",
-                causal_conv1d_implementation="eager", chunk_gated_delta_rule_implementation="eager")
-    base.update(kw)
-    return cls(**base)
-
-
-def _batch(dev, vocab):
-    lens = [300, 212, 512]
-    g = torch.Generator().manual_seed(11)
-    ids = torch.randint(0, vocab, (1, sum(lens)), generator=g)
-    labels = ids.clone()
-    off = 0
-    for n in lens:
-        labels[0, off] = -100
-        off += n
-    pos = torch.cat([torch.arange(n) for n in lens])[None]
-    cu = torch.tensor([0] + list(torch.tensor(lens).cumsum(0)), dtype=torch.int32)
-    return dict(input_ids=ids.to(dev), labels=labels.to(dev), position_ids=pos.to(dev), attention_mask=torch.ones_like(ids).to(dev),
-                cu_seq_lens_q=cu.to(dev), cu_seq_lens_k=cu.to(dev), max_length_q=max(lens), max_length_k=max(lens))
-
-
-def _run(build, cfg_dict, ops, dev, state=None):
-    with tempfile.TemporaryDirectory() as d:
-        (Path(d) / "config.json").write_text(json.dumps(cfg_dict))
-        torch.manual_seed(0)
-        model = build(config_path=d, weights_path=None, torch_dtype="bfloat16", init_device="cuda", ops_implementation=ops)
-    if state is None:
-        torch.manual_seed(0)
-        model.init_weights()
-        state = {k: v.detach().clone() for k, v in model.state_dict().items()}
-    else:
-        model.load_state_dict(state)
-    model.train()
-    out = model(**_batch(dev, cfg_dict["vocab_size"]), use_cache=False)
-    out.loss.backward()
-    gn = torch.sqrt(sum((p.grad.float() ** 2).sum() for p in model.parameters() if p.grad is not None))
-    return float(out.loss.detach()), float(gn), state
-
-
-@pytest.mark.parametrize("name,cfg", [("qwen3", QWEN3_TOY), ("qwen3_moe", QWEN3_MOE_TOY)])
+@pytest.mark.parametrize("name,cfg", CASES)
 def test_reference_models_with_b200_ops_match_reference_stock_ops(cuda_dev, name, cfg):
-    build, Ops = _reference()
+    if not (REF_DIR / "veomni").is_dir():
+        pytest.skip("oracle/_ref holds no reference package (build() found no reference source)")
     from veomni_b200 import _lib, registry
 
-    assert registry.register(), "veomni_b200.registry.register() found no importable VeOmni"
-    stock = _ops(Ops)  # reference eager ops + its stock flash-attn-2 varlen attention
-    loss_ref, gn_ref, state = _run(build, cfg, stock, cuda_dev)
+    sys.path.insert(0, str(REF_DIR))
+    try:
+        assert registry.register(), "veomni_b200.registry.register() found no importable VeOmni"
+        _lib.reset_launch_count()
+        res = MRB.reference_run(cfg, cuda_dev, attn_implementation=registry.ATTN_NAME, rms_norm_implementation="b200",
+                                rotary_pos_emb_implementation="b200", swiglu_mlp_implementation="b200",
+                                cross_entropy_loss_implementation="b200",
+                                moe_implementation="fused_b200" if name == "qwen3_moe" else "eager")
+    finally:
+        sys.path.remove(str(REF_DIR))
+    _check(name, res["loss"], res["grad_norm"], _lib.launch_count())
+
+
+@pytest.mark.parametrize("name,cfg", CASES)
+def test_host_models_match_reference_stock_ops(cuda_dev, name, cfg):
+    from veomni_b200 import _lib
+
+    model = MRB.toy_model(cfg).to(cuda_dev).to(torch.bfloat16)
+    model.train()
+    ids, labels, lens = MRB.toy_batch(cfg["vocab_size"])
+    pos = torch.cat([torch.arange(n) for n in lens])[None]
+    cu = torch.tensor([0] + list(torch.tensor(lens).cumsum(0)), dtype=torch.int32, device=cuda_dev)
     _lib.reset_launch_count()
-    b200 = _ops(Ops, attn_implementation=registry.ATTN_NAME, rms_norm_implementation="b200", rotary_pos_emb_implementation="b200",
-                swiglu_mlp_implementation="b200", cross_entropy_loss_implementation="b200",
-                moe_implementation="fused_b200" if name == "qwen3_moe" else "eager")
-    loss, gn, _ = _run(build, cfg, b200, cuda_dev, state)
-    assert _lib.launch_count() > 0, "the b200 arm did not launch a single veomni_b200 kernel"
-    print(json.dumps({"model": name, "loss_ref": loss_ref, "loss_b200": loss, "grad_norm_ref": gn_ref, "grad_norm_b200": gn,
-                      "b200_kernel_launches": _lib.launch_count()}))
-    assert abs(loss - loss_ref) / abs(loss_ref) < 1e-2, (loss, loss_ref)
-    assert abs(gn - gn_ref) / gn_ref < 1e-2, (gn, gn_ref)
+    loss = model(ids.to(cuda_dev), pos.to(cuda_dev), cu, max(lens), labels=labels.to(cuda_dev))
+    loss.backward()
+    gn = torch.sqrt(sum((p.grad.float() ** 2).sum() for p in model.parameters() if p.grad is not None))
+    _check(name, float(loss.detach()), float(gn), _lib.launch_count())

@@ -44,13 +44,14 @@ def test_duplicate_registration_rejected():
 
 
 def test_register_into_the_real_reference_when_present():
-    """In the authoring container the reference tree is importable: the b200 kernels land in ITS registry."""
-    import os
+    """With the reference package built into oracle/_ref (oracle/build_ref.py), the b200 kernels land in ITS registry."""
     import sys
 
-    if not os.path.isdir("/root/reference/veomni"):
-        pytest.skip("reference tree not present (GPU box)")
-    sys.path.insert(0, "/root/reference")
+    from oracle.build_ref import REF_DIR
+
+    if not (REF_DIR / "veomni").is_dir():
+        pytest.skip("oracle/_ref holds no reference package (build() found no reference source)")
+    sys.path.insert(0, str(REF_DIR))
     try:
         assert R.register() is True
         from transformers.modeling_utils import ALL_ATTENTION_FUNCTIONS
@@ -71,4 +72,4 @@ def test_register_into_the_real_reference_when_present():
 
         assert u.all_to_all_tensor.__module__ == "veomni_b200.ulysses"
     finally:
-        sys.path.remove("/root/reference")
+        sys.path.remove(str(REF_DIR))
