@@ -151,6 +151,33 @@ int vb200_cross_entropy(const void* logits, int32_t dtype, int64_t rows, int64_t
                         const int64_t* labels, int64_t ignore_index, float* loss_rows, float* lse,
                         int32_t lse_given, void* grad, int64_t grad_stride, float scale,
                         const float* scale_dev, const float* upstream, void* stream);
+/* ---- per-token log-probs, entropy and top-k forward-KL distillation -------------------------
+ * Replaces the arithmetic of _ChunkedLinearLogProbs (veomni/ops/kernels/cross_entropy/chunk_logprobs.py:126-268)
+ * and _ChunkedLinearTopkDistill (chunk_topk_distill.py:79-326) on one logits chunk, as reached through
+ * ForCausalLMLoss(return_log_probs=True) (__init__.py:130-177).
+ *   logits [rows, vocab], dtype 0 = bf16, 1 = f32, row stride in elements; rows, vocab < 2^31
+ *   x = round_dtype(logits / temperature) (a true division in fp32, then rounded: chunk_logprobs.py:173-176)
+ *   lse[r] = logsumexp(x_r) (may be NULL); logp[r] = x_r[label_r] - lse[r]; entropy[r] = lse[r] - sum softmax(x_r) x_r
+ *   k = 0: no distillation. 0 < k <= 1024: topk_ids [rows, k] int64, topk_logp [rows, k] (topk_dtype 0 = bf16,
+ *   1 = f32) and   slp = x[id] - lse,  student_mass = sum exp(slp),  teacher_mass = sum exp(tlp),
+ *                  distill = sum exp(tlp') (tlp' - slp'),  ' = max(., clamp) when has_clamp
+ *   Every output is 0 where label == ignore_index; logp is NaN for a label outside [0, vocab).           */
+int vb200_token_logprobs(const void* logits, int32_t dtype, int64_t rows, int64_t vocab, int64_t row_stride,
+                         const int64_t* labels, int64_t ignore_index, float temperature, float* lse, float* logp,
+                         float* entropy, int32_t k, const int64_t* topk_ids, const void* topk_logp, int32_t topk_dtype,
+                         int32_t has_clamp, float clamp, float* distill, float* student_mass, float* teacher_mass,
+                         void* stream);
+/* Gradient of sum_r dlogp[r] logp[r] + dentropy[r] entropy[r] + ddistill[r] distill[r] w.r.t. the logits
+ * (chunk_logprobs.py:230-258, chunk_topk_distill.py:252-313), written to grad (same dtype; may alias logits).
+ * lse / entropy are the forward's outputs; each upstream pointer may be NULL (= 0). With p = softmax(x):
+ *   g_v = dlogp (d(v=label) - p_v) - dentropy p_v (x_v - lse + entropy)
+ *         + ddistill (teacher_mass_eff p_v - pt[v]),  pt[v] = sum_{k: id_k = v} exp(tlp'_k) [slp_k >= clamp],
+ *   teacher_mass_eff = sum_v pt[v];  grad = round_dtype(round_dtype(g) / temperature).  0 at ignored rows. */
+int vb200_token_logprobs_bwd(const void* logits, int32_t dtype, int64_t rows, int64_t vocab, int64_t row_stride,
+                             const int64_t* labels, int64_t ignore_index, float temperature, const float* lse,
+                             const float* entropy, const float* dlogp, const float* dentropy, const float* ddistill,
+                             int32_t k, const int64_t* topk_ids, const void* topk_logp, int32_t topk_dtype,
+                             int32_t has_clamp, float clamp, void* grad, int64_t grad_stride, void* stream);
 /* out2[0] = 1 / count(labels != ignore_index) (0 if none), out2[1] = that count; device scalars. */
 int vb200_count_valid_labels(const int64_t* labels, int64_t n, int64_t ignore_index, float* out2,
                              void* stream);

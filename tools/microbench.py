@@ -228,6 +228,62 @@ def bench_loss(dev, iters):
     del g32, lr
 
 
+def bench_logprobs(dev, iters):
+    """Per-token log-probs / entropy / top-k distillation (token_stats_kernel, token_grad_kernel) on one 1024-row chunk of
+    the 151936-entry vocabulary in bf16, without and with K = 64 teacher entries; then the fused-linear forward + backward
+    at T = H = 4096 against the oracle's torch restatement of the reference arithmetic on the same CUDA tensors."""
+    from oracle import logprobs as O
+    from veomni_b200.cross_entropy import _token_launch, chunk_topk_distill_function
+
+    rows, V, K = 1024, 151936, 64
+    f32 = dict(dtype=torch.float32, device=dev)
+    labels = torch.randint(0, V, (rows,), device=dev)
+    ids = torch.randint(0, V, (rows, K), device=dev)
+    tlp = torch.log_softmax(torch.randn(rows, K, device=dev), -1)
+    st = [torch.empty(rows, **f32) for _ in range(6)]
+    ups = [torch.randn(rows, **f32) for _ in range(3)]
+    sets = [(torch.randn(rows, V, device=dev, dtype=BF),) for _ in range(2)]  # 2 x 311 MB > L2
+    for k in (0, K):
+        kid, ktl = (ids, tlp) if k else (None, None)
+
+        def fwd(x):
+            _token_launch(False, x, labels, -100, 1.0, st[0], st[1], kid, ktl, None, logp=st[2], dist=st[3], sm=st[4], tm=st[5])
+
+        report(f"token_logprobs_fwd[1024x151936 bf16, K={k}]", time_fn(fwd, sets, iters), nbytes=rows * V * 2)
+        fwd(sets[0][0])
+
+        def bwd(x):  # in place; the values drift between calls, the traffic does not
+            _token_launch(True, x, labels, -100, 1.0, st[0], st[1], kid, ktl, None, ups=ups if k else ups[:2] + [None])
+
+        report(f"token_logprobs_grad_inplace[1024x151936 bf16, K={k}]", time_fn(bwd, sets, iters), nbytes=2 * rows * V * 2)
+    del sets
+    T, H = 4096, 4096
+    h = (torch.randn(T, H, device=dev) * 0.5).to(BF).requires_grad_(True)
+    w = (torch.randn(V, H, device=dev) * 0.02).to(BF).requires_grad_(True)
+    lab = torch.randint(0, V, (T,), device=dev)
+    tids = torch.randint(0, V, (T, K), device=dev)
+    ttlp = torch.log_softmax(torch.randn(T, K, device=dev), -1)
+    up = [torch.randn(T, **f32) for _ in range(3)]
+
+    def ours():
+        outs = chunk_topk_distill_function(h, w, lab, tids, ttlp, shift_labels=lab)
+        torch.autograd.grad(sum((o * u).sum() for o, u in zip(outs[:3], up)), (h, w))
+
+    def eager():  # the reference's per-chunk arithmetic: fp32 [1024, V] softmax / log_softmax / dense teacher temporaries
+        with torch.no_grad():
+            O.fused_linear_token_logprobs(h, w, lab, tids, ttlp, upstream=up)
+
+    for name, fn in (("chunk_topk_distill fwd+bwd (veomni_b200)", ours), ("(oracle) eager restatement fwd+grads", eager)):
+        fn()
+        torch.cuda.synchronize()
+        torch.cuda.reset_peak_memory_stats(dev)
+        base = torch.cuda.memory_allocated(dev)
+        us = time_fn(lambda: fn(), [()], max(3, iters // 10), warmup=1)
+        r = {"kernel": f"{name}[T=4096 H=4096 V=151936 K=64 bf16]", "ms": round(us / 1e3, 2),
+             "peak_extra_GB": round((torch.cuda.max_memory_allocated(dev) - base) / 1e9, 2)}
+        print(json.dumps(r), flush=True)
+
+
 def bench_fsdp(dev, iters):
     """FSDP2 copy-in kernels and the gradient-clip kernels at Qwen3-8B layer-unit sizes (193 M parameters per unit)."""
     import ctypes
@@ -279,7 +335,8 @@ def bench_fsdp(dev, iters):
     report("(lib) torch._foreach_mul_", time_fn(lambda: torch._foreach_mul_(big, coef), [()], iters), nbytes=8 * tot)
 
 
-BENCHES = {"rmsnorm": bench_rmsnorm, "rope": bench_rope, "swiglu": bench_swiglu, "loss": bench_loss, "fsdp": bench_fsdp}
+BENCHES = {"rmsnorm": bench_rmsnorm, "rope": bench_rope, "swiglu": bench_swiglu, "loss": bench_loss, "logprobs": bench_logprobs,
+           "fsdp": bench_fsdp}
 
 
 def main():

@@ -52,6 +52,10 @@ SIGNATURES = {
     "vb200_multi_adamw": (c_int, [_P, _P, _P, _P, _P, _P, _I32, _I32, _F, _F, _F, _F, _F, _F, _F, _P, _P]),
     "vb200_cross_entropy": (c_int, [_P, _I32, _I64, _I64, _I64, _P, _I64, _P, _P, _I32, _P, _I64, _F, _P, _P, _P]),
     "vb200_count_valid_labels": (c_int, [_P, _I64, _I64, _P, _P]),
+    "vb200_token_logprobs": (c_int, [_P, _I32, _I64, _I64, _I64, _P, _I64, _F, _P, _P, _P, _I32, _P, _P, _I32, _I32, _F,
+                                     _P, _P, _P, _P]),
+    "vb200_token_logprobs_bwd": (c_int, [_P, _I32, _I64, _I64, _I64, _P, _I64, _F, _P, _P, _P, _P, _P, _I32, _P, _P,
+                                         _I32, _I32, _F, _P, _I64, _P]),
     "vb200_swiglu_fwd": (c_int, [_P, _P, _P, _I64, _I64, _I64, _I64, _P]),
     "vb200_swiglu_bwd": (c_int, [_P] * 5 + [_I64] * 5 + [_P]),
     "vb200_attn_varlen_fwd": (c_int, [_P] * 6 + [_I32] * 6 + [_P, _F, _I32, _P]),

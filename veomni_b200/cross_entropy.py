@@ -9,12 +9,16 @@ Mirrors veomni/ops/kernels/cross_entropy/:
   the CUDA kernel turns each logits chunk into its gradient in place, and the full ``[T, V]`` logits (2.5 GB in
   fp32 at T=4096, V=151936) never exist.
 * :func:`ForCausalLMLoss` is the outer policy (__init__.py:89-221): label shift unless SP, flatten, SP loss reduce.
+* :func:`chunk_logprobs_function` / :func:`chunk_topk_distill_function` are the ``return_log_probs=True`` paths
+  (chunk_logprobs.py, chunk_topk_distill.py): per-token log-probs and entropy, and top-k forward-KL distillation,
+  through the same chunked lm_head; each logits chunk is turned into its gradient in place in backward.
 
 No host synchronisation: the valid-token count stays on the device and scales loss and gradient there.
 """
 
 from __future__ import annotations
 
+from dataclasses import dataclass
 from typing import Any, Callable
 
 import torch
@@ -147,6 +151,198 @@ class _FusedLinearCrossEntropy(torch.autograd.Function):
         return gh, gw, None, None, None, None, None
 
 
+class _FusedLinearTokenLogProbs(torch.autograd.Function):
+    """lm_head projection + per-token log-probs and entropy, plus top-k forward-KL distillation when ``ids`` is given
+    (K = ids.size(1) > 0): the arithmetic of _ChunkedLinearLogProbs / _ChunkedLinearTopkDistill
+    (chunk_logprobs.py:126-268, chunk_topk_distill.py:79-326), chunked over rows.
+
+    Forward: per chunk, logits on cuBLAS, then ``token_stats_kernel``; only the fp32 ``[T]`` statistics are kept.
+    Backward: per chunk, the same GEMM recomputes the logits, ``token_grad_kernel`` turns them into dlogits in place,
+    and two GEMMs give dh and dw. The weight saved here is the lm_head parameter, which FSDP2's pre-backward hook has
+    unsharded again by the time backward runs (the reference's contract, chunk_logprobs.py:42-48).
+    Outputs: ``(logp, entropy)``, or with K > 0 ``(logp, entropy, distill, student_mass, teacher_mass)``, the last
+    two non-differentiable."""
+
+    @staticmethod
+    def forward(ctx: Any, hidden: torch.Tensor, weight: torch.Tensor, labels: torch.Tensor, ids: torch.Tensor | None,
+                tlp: torch.Tensor | None, temperature: float, chunk_size: int, ignore_index: int, clamp: float | None):
+        ctx.set_materialize_grads(False)
+        _check_token_inputs(hidden, weight, labels, ids, tlp)
+        T, dev = hidden.size(0), hidden.device
+        K = ids.size(1) if ids is not None else 0
+        f32 = dict(dtype=torch.float32, device=dev)
+        lse, logp, ent = torch.empty(T, **f32), torch.empty(T, **f32), torch.empty(T, **f32)
+        dist, sm, tm = (torch.empty(T, **f32) for _ in range(3)) if K else (None, None, None)
+        wt = weight.t()
+        for r0 in range(0, T, chunk_size):
+            r1 = min(T, r0 + chunk_size)
+            logits = torch.mm(hidden[r0:r1], wt)  # [chunk, V] in the compute dtype (cuBLAS)
+            _token_launch(False, logits, labels[r0:r1], ignore_index, temperature, lse[r0:r1], ent[r0:r1],
+                          ids[r0:r1] if K else None, tlp[r0:r1] if K else None, clamp,
+                          logp=logp[r0:r1], dist=dist[r0:r1] if K else None, sm=sm[r0:r1] if K else None,
+                          tm=tm[r0:r1] if K else None)
+        ctx.save_for_backward(hidden, weight, labels, lse, ent, ids, tlp)
+        ctx.temperature, ctx.chunk_size, ctx.ignore_index, ctx.clamp = temperature, chunk_size, ignore_index, clamp
+        if not K:
+            return logp, ent
+        ctx.mark_non_differentiable(sm, tm)
+        return logp, ent, dist, sm, tm
+
+    @staticmethod
+    def backward(ctx: Any, *grads):
+        ups = list(grads[:3]) + [None] * (3 - len(grads[:3]))  # dlogp, dentropy, ddistill (absent for K = 0)
+        nones = (None,) * 9
+        if all(g is None for g in ups):
+            return nones
+        hidden, weight, labels, lse, ent, ids, tlp = ctx.saved_tensors
+        need_h, need_w = ctx.needs_input_grad[0], ctx.needs_input_grad[1]
+        if not (need_h or need_w):
+            return nones
+        ups = [g.detach().reshape(-1).to(torch.float32).contiguous() if g is not None else None for g in ups]
+        K = ids.size(1) if ids is not None else 0
+        grad_h = torch.empty_like(hidden) if need_h else None
+        grad_w = torch.zeros_like(weight) if need_w else None
+        wt = weight.t()
+        cs = ctx.chunk_size
+        for r0 in range(0, hidden.size(0), cs):
+            r1 = min(hidden.size(0), r0 + cs)
+            h_c = hidden[r0:r1]
+            logits = torch.mm(h_c, wt)
+            _token_launch(True, logits, labels[r0:r1], ctx.ignore_index, ctx.temperature, lse[r0:r1], ent[r0:r1],
+                          ids[r0:r1] if K else None, tlp[r0:r1] if K else None, ctx.clamp,
+                          ups=[u[r0:r1] if u is not None else None for u in ups])  # logits now hold dlogits
+            if need_h:
+                torch.mm(logits, weight, out=grad_h[r0:r1])
+            if need_w:
+                grad_w.addmm_(logits.t(), h_c)
+        return (grad_h, grad_w) + nones[2:]
+
+
+def _check_token_inputs(hidden, weight, labels, ids, tlp) -> None:
+    if not (hidden.is_cuda and weight.is_cuda and labels.is_cuda):
+        raise VB200Error("token log-probs run on CUDA tensors only (no CPU fallback)")
+    if hidden.dim() != 2 or weight.dim() != 2 or hidden.size(1) != weight.size(1):
+        raise VB200Error("token log-probs: hidden [T, H] and weight [V, H] expected")
+    if hidden.dtype != weight.dtype or hidden.dtype not in _DT:
+        raise VB200Error("token log-probs: hidden states and weights must share a dtype, bf16 or fp32")
+    if labels.dtype != torch.int64 or labels.shape != (hidden.size(0),):
+        raise VB200Error("token log-probs: labels must be int64 [T]")
+    if ids is None:
+        return
+    if not (ids.is_cuda and tlp.is_cuda):
+        raise VB200Error("token log-probs: teacher top-k tensors must be CUDA tensors")
+    if ids.dtype != torch.int64 or ids.dim() != 2 or ids.size(0) != hidden.size(0) or tlp.shape != ids.shape:
+        raise VB200Error("token log-probs: teacher_topk_ids int64 [T, K] and teacher_topk_log_probs [T, K] expected")
+    if tlp.dtype not in _DT:
+        raise VB200Error(f"token log-probs: teacher log-probs must be bf16 or fp32, got {tlp.dtype}")
+    if not (ids.is_contiguous() and tlp.is_contiguous()):
+        raise VB200Error("token log-probs: teacher top-k tensors must be contiguous")
+
+
+def _token_launch(backward: bool, logits, labels, ignore_index, temperature, lse, ent, ids, tlp, clamp,
+                  logp=None, dist=None, sm=None, tm=None, ups=None) -> None:
+    """One ``vb200_token_logprobs`` (forward) or ``vb200_token_logprobs_bwd`` (backward, in place) call on a chunk."""
+    _check(logits, labels)
+    lib = _lib.load()
+    K = ids.size(1) if ids is not None else 0
+    topk = (K, _ptr(ids), _ptr(tlp), _DT[tlp.dtype] if K else 0, int(clamp is not None),
+            float(clamp) if clamp is not None else 0.0)
+    head = (logits.data_ptr(), _DT[logits.dtype], logits.size(0), logits.size(1), logits.stride(0), labels.data_ptr(),
+            int(ignore_index), float(temperature))
+    with torch.cuda.device(logits.device):
+        if backward:
+            check(lib.vb200_token_logprobs_bwd(*head, lse.data_ptr(), ent.data_ptr(), *map(_ptr, ups), *topk,
+                                               logits.data_ptr(), logits.stride(0), stream_ptr()),
+                  "vb200_token_logprobs_bwd")
+        else:
+            check(lib.vb200_token_logprobs(*head, lse.data_ptr(), logp.data_ptr(), ent.data_ptr(), *topk, _ptr(dist),
+                                           _ptr(sm), _ptr(tm), stream_ptr()), "vb200_token_logprobs")
+
+
+def _shift_for_logprobs(hidden_states, labels, shift_labels, sp_enabled, teacher=()):
+    """The target choice of chunk_logprobs.py:319-338 / chunk_topk_distill.py:379-393: explicit ``shift_labels`` as
+    given; SP already shifted by the collator; otherwise ``labels[..., 1:]`` against ``hidden[..., :-1, :]`` (and the
+    teacher tensors shifted with the labels). Returns (hidden, labels, teacher tensors, pad the outputs?)."""
+    if shift_labels is not None:
+        return hidden_states, shift_labels, teacher, False
+    if sp_enabled:
+        return hidden_states, labels, teacher, False
+    return hidden_states[..., :-1, :], labels[..., 1:], tuple(t[..., 1:, :] for t in teacher), True
+
+
+def _token_logprobs(hidden_states, weights, labels, teacher, chunk_size, ignore_index, temperature, clamp, pad):
+    if not (hidden_states.is_cuda and weights.is_cuda and labels.is_cuda):
+        raise VB200Error("token log-probs run on CUDA tensors only (no CPU fallback)")
+    shape = labels.shape
+    h = hidden_states.reshape(-1, hidden_states.size(-1))
+    lab = labels.reshape(-1).to(torch.int64)
+    ids = tlp = None
+    if teacher:
+        K = teacher[0].size(-1)
+        ids = teacher[0].reshape(-1, K).to(torch.int64).contiguous()
+        tlp = teacher[1].reshape(-1, K).contiguous()
+    outs = _FusedLinearTokenLogProbs.apply(h, weights, lab, ids, tlp, float(temperature), int(chunk_size),
+                                           int(ignore_index), None if clamp is None else float(clamp))
+    outs = [o.view(shape) for o in outs]
+    if pad:  # the final input token has no next-token target: one zero slot keeps the shape of ``labels``
+        outs = [F.pad(o, (0, 1), value=0.0) for o in outs]
+    if teacher:
+        outs[3], outs[4] = outs[3].detach(), outs[4].detach()
+    return tuple(outs)
+
+
+def chunk_logprobs_function(
+    hidden_states: torch.Tensor,
+    weights: torch.Tensor,
+    labels: torch.Tensor,
+    chunk_size: int = 1024,
+    ignore_index: int = -100,
+    shift_labels: torch.Tensor | None = None,
+    temperature: float = 1.0,
+    *,
+    sp_enabled: bool = False,
+) -> tuple[torch.Tensor, torch.Tensor]:
+    """Per-token ``log p(label)`` and softmax entropy through the chunked lm_head, without the ``[T, V]`` logits
+    (the contract of chunk_logprobs.py:271-351). Both outputs have the shape of ``labels`` and are 0 at ignored
+    positions; without ``shift_labels`` and SP the causal shift is applied here and the last slot is 0.
+    ``sp_enabled`` stands for the reference's global parallel state: labels already shifted by the SP collator."""
+    h, lab, _, pad = _shift_for_logprobs(hidden_states, labels, shift_labels, sp_enabled)
+    return _token_logprobs(h, weights, lab, (), chunk_size, ignore_index, temperature, None, pad)
+
+
+def chunk_topk_distill_function(
+    hidden_states: torch.Tensor,
+    weights: torch.Tensor,
+    labels: torch.Tensor,
+    teacher_topk_ids: torch.Tensor,
+    teacher_topk_log_probs: torch.Tensor,
+    chunk_size: int = 1024,
+    ignore_index: int = -100,
+    shift_labels: torch.Tensor | None = None,
+    temperature: float = 1.0,
+    log_prob_min_clamp: float | None = None,
+    *,
+    sp_enabled: bool = False,
+) -> tuple[torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor]:
+    """``(log_probs, entropy, distillation_losses, student_mass, teacher_mass)`` of the top-k forward KL
+    (chunk_topk_distill.py:329-416): ``teacher_topk_ids`` int64 ``[..., K]`` (K <= 1024) and
+    ``teacher_topk_log_probs`` bf16 / fp32 ``[..., K]`` aligned with ``labels``. The two masses are detached."""
+    h, lab, teacher, pad = _shift_for_logprobs(hidden_states, labels, shift_labels, sp_enabled,
+                                               (teacher_topk_ids, teacher_topk_log_probs))
+    return _token_logprobs(h, weights, lab, teacher, chunk_size, ignore_index, temperature, log_prob_min_clamp, pad)
+
+
+@dataclass
+class FusedLinearAuxOutput:
+    """Per-token tensors of the log-probs paths; the field names of veomni.utils.model_outputs.FusedLinearAuxOutput."""
+
+    log_probs: torch.Tensor | None = None
+    entropy: torch.Tensor | None = None
+    distillation_losses: torch.Tensor | None = None
+    student_mass: torch.Tensor | None = None
+    teacher_mass: torch.Tensor | None = None
+
+
 class _ReduceLoss(torch.autograd.Function):
     """Token-weighted mean of the per-rank losses over the SP group (sequence_parallel/loss.py:27-60):
     forward sum_r(loss_r * n_r) / max(sum_r n_r, 1), a rank without valid tokens contributing 0;
@@ -211,9 +407,18 @@ def ForCausalLMLoss(
     """Outer policy of the causal-LM loss (reference __init__.py:89-221, loss path only): shift labels unless the
     sequence is SP-sharded (then the data pipeline already shifted them), flatten, call the kernel, and reduce the
     loss over the SP group weighted by each rank's valid-token count (sequence_parallel/loss.py).
-    Returns ``(loss, logits, None)`` like the reference wrapper."""
+    Returns ``(loss, logits, None)`` like the reference wrapper.
+
+    With ``return_log_probs=True`` (reference __init__.py:107-177) the loss path is skipped: the per-token tensors of
+    :func:`chunk_logprobs_function`, or of :func:`chunk_topk_distill_function` when ``teacher_topk_ids`` and
+    ``teacher_topk_log_probs`` are passed, come back as ``(None, None, FusedLinearAuxOutput)``. ``temperature``,
+    ``log_prob_min_clamp`` and ``chunk_size`` are forwarded to them."""
     hidden_states = kwargs.pop("hidden_states", None)
     weights = kwargs.pop("weights", None)
+    if kwargs.pop("return_log_probs", False):
+        sp_enabled = sp_group is not None and torch.distributed.get_world_size(sp_group) > 1
+        return None, None, _log_probs_branch(hidden_states, weights, labels, ignore_index, shift_labels, sp_enabled,
+                                             **kwargs)
     if hidden_states is None and logits is None:
         raise VB200Error("hidden_states or logits must be provided.")
     sp_enabled = sp_group is not None and torch.distributed.get_world_size(sp_group) > 1
@@ -233,3 +438,25 @@ def ForCausalLMLoss(
     if sp_enabled:
         loss = _ReduceLoss.apply(loss, (shift_labels != ignore_index).sum(), sp_group)
     return loss, logits, None
+
+
+def _log_probs_branch(hidden_states, weights, labels, ignore_index, shift_labels, sp_enabled, temperature=1.0,
+                      teacher_topk_ids=None, teacher_topk_log_probs=None, log_prob_min_clamp=None, chunk_size=1024,
+                      **_ignored) -> FusedLinearAuxOutput:
+    """The ``return_log_probs=True`` branch of ForCausalLMLoss, with the reference's errors (__init__.py:135-143)."""
+    if hidden_states is None:
+        raise ValueError("return_log_probs=True requires hidden_states (fused-linear path).")
+    if weights is None:
+        raise ValueError("return_log_probs=True requires weights (lm_head weight).")
+    if (teacher_topk_ids is None) != (teacher_topk_log_probs is None):
+        raise ValueError("teacher_topk_ids and teacher_topk_log_probs must be provided together for "
+                         "the top-k distillation path.")
+    common = dict(chunk_size=chunk_size, ignore_index=ignore_index, shift_labels=shift_labels, temperature=temperature,
+                  sp_enabled=sp_enabled)
+    if teacher_topk_ids is not None:
+        lp, ent, dist, sm, tm = chunk_topk_distill_function(hidden_states, weights, labels, teacher_topk_ids,
+                                                            teacher_topk_log_probs, log_prob_min_clamp=log_prob_min_clamp,
+                                                            **common)
+        return FusedLinearAuxOutput(log_probs=lp, entropy=ent, distillation_losses=dist, student_mass=sm, teacher_mass=tm)
+    lp, ent = chunk_logprobs_function(hidden_states, weights, labels, **common)
+    return FusedLinearAuxOutput(log_probs=lp, entropy=ent)

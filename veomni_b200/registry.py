@@ -191,6 +191,32 @@ for _s in _specs():
     KERNEL_REGISTRY.register(_s, force=True)
 
 
+def _token_fn_dispatcher(name: str, orig: Callable) -> Callable:
+    """Stand-in for the reference's ``chunk_logprobs_function`` / ``chunk_topk_distill_function`` (``name``): when the
+    installed ops config selects ``cross_entropy_loss_implementation == "b200"``, the call goes to the function of the
+    same name in :mod:`veomni_b200.cross_entropy`, with ``sp_enabled`` read from the reference's parallel state;
+    otherwise to ``orig``, unchanged. The selection is process-global, like ``LOSS_MAPPING`` and the shared OpSlots:
+    the ops config in force at call time decides. ``orig`` stays reachable as ``_vb200_orig``."""
+
+    def dispatch(*args, **kwargs):
+        from veomni.ops.config.singleton import get_ops_config
+
+        cfg = get_ops_config()
+        if cfg is not None and getattr(cfg, "cross_entropy_loss_implementation", None) == IMPL_NAME:
+            from veomni.distributed.parallel_state import get_parallel_state
+
+            from . import cross_entropy as own
+
+            return getattr(own, name)(*args, sp_enabled=get_parallel_state().sp_enabled, **kwargs)
+        return dispatch._vb200_orig(*args, **kwargs)
+
+    dispatch.__name__ = dispatch.__qualname__ = name
+    dispatch.__doc__ = orig.__doc__
+    dispatch._vb200 = True
+    dispatch._vb200_orig = orig
+    return dispatch
+
+
 def register(force: bool = True) -> bool:
     """Plug the kernels into an installed VeOmni. Returns False (and does nothing) if it is not importable."""
     try:
@@ -232,6 +258,17 @@ def register(force: bool = True) -> bool:
 
             _resolve_cross_entropy_fn._vb200 = True
             ref_ce._resolve_cross_entropy_fn = _resolve_cross_entropy_fn
+    except Exception:  # noqa: BLE001
+        pass
+    # per-token log-probs / top-k distillation: ForCausalLMLoss and _chunk_loss_dispatch call these module globals
+    # when the caller passes return_log_probs=True (veomni/ops/kernels/cross_entropy/__init__.py:130-177,395-439)
+    try:
+        import veomni.ops.kernels.cross_entropy as ref_ce
+
+        for name in ("chunk_logprobs_function", "chunk_topk_distill_function"):
+            fn = getattr(ref_ce, name)
+            if not getattr(fn, "_vb200", False):
+                setattr(ref_ce, name, _token_fn_dispatcher(name, fn))
     except Exception:  # noqa: BLE001
         pass
     # fused MoE raw pointer (veomni/ops/kernels/moe/__init__.py:62-108)
